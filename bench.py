@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # GPU arm (libvlscan.so)
     python bench.py --impl reference [--gpus N] [--steps K] ...    # reference arm: the CPU algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                         # also write what the last timed step computed to DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic blocks:  bm.init/setBits + filter.applyToBlockSearch for every
 block (lib/logstorage/block_search.go:207-215).
@@ -70,7 +71,14 @@ def parse_args():
     ap.add_argument("--cpu-sample-rows", type=int, default=12_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra workloads (C2, C4) measured next to the headline at N=1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (rank 0's shard) as DIR/<name>.npy, "
+                    "so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "vlscan":
+        ap.error("--dump-outputs writes the device scan's outputs: --impl vlscan only")
+    return args
 
 
 class ClockSampler:
@@ -195,15 +203,12 @@ def run_reference(args, wl, gen_kw, rank, world):
     if rank != 0:
         return
     threads = os.cpu_count() or 1
-    t0 = time.time()
     rates, info = [], None
-    n = args.warmup + max(args.steps, 5)
+    n = args.warmup + args.steps
     for i in range(n):
         rate, info = cpu_port(wl, gen_kw, args.cpu_sample_rows, threads, target_secs=min(8.0, 160.0 / n))
         if i >= args.warmup:
             rates.append(rate)
-        if time.time() - t0 > 200 and len(rates) >= 3:
-            break
     value = statistics.median(rates)
     hi = host_info()
     out = {
@@ -228,6 +233,25 @@ def words_digest(vloracle, words, rows_list, key_base):
         d ^= (vloracle.xxh64(words[off:off + nw].tobytes()) * (2 * (key_base + i) + 1)) & 0xFFFFFFFFFFFFFFFF
         off += nw
     return d
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, words, counts, block_rows):
+    """What a caller of the resident scan receives, as float arrays of at most DUMP_BYTES in all: the match count of every block
+    (block_match_counts), and the per-row match bits (0 / 1, block after block) of a fixed, seeded sample of the blocks (sample_match_bits)
+    whose indices are sample_blocks - every block when the bitmaps fit.  The bits of a block are its bitmap words, least significant first."""
+    import numpy as np
+    nb = len(block_rows)
+    word_off = np.concatenate(([0], np.cumsum((block_rows + 63) // 64)))
+    k = min(nb, (DUMP_BYTES - 8 * nb - 4096) // (4 * int(block_rows.max()) + 8))
+    pick = np.sort(np.random.default_rng(SEED).choice(nb, size=k, replace=False))
+    bits = [np.unpackbits(words[word_off[b]:word_off[b + 1]].view(np.uint8), bitorder="little")[:block_rows[b]] for b in pick]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "block_match_counts.npy"), counts.astype(np.float64))
+    np.save(os.path.join(out_dir, "sample_blocks.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "sample_match_bits.npy"), np.concatenate(bits).astype(np.float32))
 
 
 def main():
@@ -276,8 +300,9 @@ def main():
         torch.cuda.synchronize()
         ctx.sync()
 
-    def measure(w, w_rows, w_nb, w_kw, steps, warmup, sample_clocks):
-        """resident scan of one workload -> dict; the batch stays alive in the returned dict until the caller frees it"""
+    def measure(w, w_rows, w_nb, w_kw, steps, warmup, sample_clocks, capture=False):
+        """resident scan of one workload -> dict; the batch stays alive in the returned dict until the caller frees it.
+        capture: also return the bitmap words and match counts of the last timed step (`outputs`)"""
         gcfg = vs.GenConfig(**w_kw)
         block_lo = rank * w_nb
         t_gen = time.time()
@@ -311,6 +336,7 @@ def main():
                 shard.reduce_counters(acc)     # the only collective of the path: ONE final NCCL reduce of the match counters
         ev1.record(stream)
         sync_all()
+        outputs = ctx.fetch(batch) if capture else None   # before any untimed scan below replaces the result
         clocks = None
         if sampler:
             # the timed region may be shorter than a few nvidia-smi sampling periods: keep the same load running (untimed) until the sampler
@@ -339,7 +365,7 @@ def main():
         step_bytes = st.values_bytes + st.bloom_probe_bytes + st.bitmap_bytes
         return dict(batch=batch, prog=prog, gcfg=gcfg, block_lo=block_lo, ms=ms, steps=steps, st=st, clocks=clocks, t_gen=t_gen, k_avg=k_avg, kbytes=kbytes, achieved=achieved,
                     step_bytes=step_bytes, share=(k_avg / statistics.mean(gms)) if gms and statistics.mean(gms) > 0 else None,
-                    totals=acc.cpu().tolist() if world > 1 else None)
+                    totals=acc.cpu().tolist() if world > 1 else None, outputs=outputs)
 
     # ---- the headline workload, resident -----------------------------------------------------------------------------------------
     fallback_note = None
@@ -347,13 +373,19 @@ def main():
     want_rows = rows
     for attempt in range(4):
         try:
-            m = measure(wl, rows, nb, gen_kw, args.steps, args.warmup, True)
+            m = measure(wl, rows, nb, gen_kw, args.steps, args.warmup, True, capture=bool(args.dump_outputs) and rank == 0)
             break
         except vs.VlscanError as e:   # does not fit this GPU next to whatever else lives on it: fall back to the largest row count that does
-            if "memory" not in str(e).lower() or attempt == 3:
+            # (not when dumping: a dump must hold the outputs of the inputs the arguments name, or two dumps could not be compared)
+            if "memory" not in str(e).lower() or attempt == 3 or args.dump_outputs:
                 raise
             fallback_note = "%d rows/GPU did not fit (%s)" % (rows, str(e)[:80])
             rows, nb, gen_kw = gen_args(wl, int(rows * 0.8))
+    if m["outputs"] is not None:
+        first = m["block_lo"] * wl["rows_per_block"]
+        block_rows = np.minimum(wl["rows_per_block"], gen_kw["total_rows"] - first - wl["rows_per_block"] * np.arange(nb, dtype=np.int64))
+        dump_outputs(args.dump_outputs, *m["outputs"], block_rows)
+        m["outputs"] = None
     st, batch, prog = m["st"], m["batch"], m["prog"]
     device_bytes = batch.device_bytes
     _, resident_counts = ctx.fetch(batch, bitmaps=False, counts=True)
