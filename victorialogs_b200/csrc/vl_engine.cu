@@ -13,6 +13,7 @@
 #include <memory>
 #include <mutex>
 #include "vl_engine.h"
+#include "vl_kernels.cuh"
 #include "vl_program.h"
 #include "vl_part.h"
 #include "vl_mathnum.cuh"
@@ -157,73 +158,358 @@ static int host_threads() {
     return (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
 }
 
-// need_bloom (may be NULL = all): per batch field, whether the program that will scan this batch ever probes that field's bloom filters.  A filter
-// nobody probes stays on the host (the reference reads a column's bloom filter lazily, only when a filter asks for it: getBloomFilterForColumn,
-// block_search.go:411-439); the column is staged with an empty filter, which no kernel touches.
-//
-// mode: UP_FULL stages everything in one go.  A bloom-first upload (vlscan_scan_batch, the reference's lazy order: a column's values are read only
-// after its bloom filter let the block through, block_search.go:411-439 then :444-474) runs the function twice around the probe pass:
-// UP_HEADERS stages what the header dispatch and the bloom probes look at (const values, bloom filters, dict tables -> batch->harena) and
-// leaves every values payload on the host (VALUES_DEFERRED); UP_VALUES then stages the timestamps and the values of the columns the probe marked in
-// `need` (-> batch->arena) and flags the others VALUES_ABSENT.
-enum UploadMode { UP_FULL = 0, UP_HEADERS = 1, UP_VALUES = 2 };
-static void do_upload(vlscan_ctx* ctx, const char* const* field_names, const size_t* field_name_lens, uint32_t nfields, const vlscan_block* blocks,
-                      uint64_t nblocks, vlscan_batch* out, vlscan_stats* stats, const std::vector<char>* need_bloom = nullptr, UploadMode mode = UP_FULL,
-                      const uint8_t* need = nullptr) {
-    VL_CUDA(cudaSetDevice(ctx->device));
-    if (nblocks > 0xFFFFFFF0ull) throw BadInput("too many blocks in one batch");
-    const bool dbg = getenv("VLSCAN_DEBUG_TIMING") != nullptr;
-    auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    double t_start = now(), t_desc = 0, t_alloc = 0, t_copy = 0;
-    out->device = ctx->device; out->nfields = nfields;
-    std::vector<DevColumn>& cols = out->h_cols;   // UP_VALUES continues with the table UP_HEADERS left
-    if (mode != UP_VALUES) {
-        for (uint32_t f = 0; f < nfields; f++) out->field_names.emplace_back(field_names[f], field_name_lens[f]);
-        cols.assign((size_t)nblocks * std::max<uint32_t>(nfields, 1), DevColumn{});
-        memset(cols.data(), 0, cols.size() * sizeof(DevColumn));
-    } else if (cols.size() != (size_t)nblocks * std::max<uint32_t>(nfields, 1) || !need) throw BadInput("internal: values phase of a bloom-first upload without its header phase");
-    out->split_hdr = mode != UP_FULL;
-    DevBuf& arena_buf = mode == UP_HEADERS ? out->harena : out->arena;
-    std::vector<uint32_t> rows(nblocks);
-    struct Piece { const uint8_t* src; uint64_t len; uint64_t dst; };
-    std::vector<Piece> pieces, zpieces;   // host -> arena, host -> compressed staging (on-disk values blocks)
-    std::vector<std::unique_ptr<std::vector<uint8_t>>> owned;   // dict metadata built here
+namespace {
+// one host -> device copy: `len` bytes at host address `src` to offset `dst` of a device buffer
+struct Piece { const uint8_t* src; uint64_t len; uint64_t dst; };
+
+// The copied part of an arena: payloads reserved one behind the other (arena_reserve), each with the host bytes that go there.
+struct ArenaLayout {
     uint64_t cursor = 16;   // the first 16 bytes stay unused so that every payload has a readable byte in front of it
-    auto add_piece = [&](const uint8_t* src, uint64_t len) { uint64_t off = arena_reserve(cursor, len); if (len) pieces.push_back({src, len, off}); return off; };
-    // On-disk values blocks are not copied into the arena: their bytes go to the compressed staging buffer as they are and the device
-    // regenerates them (vl_zstd.cuh) into arena regions placed behind everything that is copied, so that host memory laid out like
-    // the copied part still goes out as one DMA.  Region offsets are relative to `regen_base` until the loop below has sized that part.
-    ZstdJob zjob;
-    uint64_t regen_cursor = 0;
+    std::vector<Piece> pieces;
+    std::vector<std::unique_ptr<std::vector<uint8_t>>> owned;   // dict tables built here
+    uint64_t put(const uint8_t* src, uint64_t len) { const uint64_t off = arena_reserve(cursor, len); if (len) pieces.push_back({src, len, off}); return off; }
+    // The header payloads of one column in their arena order: a const column's value (-> meta_off); a values column's bloom filter
+    // (-> bloom_off, `bloom_len` bytes: 0 for a filter left on the host), then for a dict column its u32 offsets[dict_len + 1] ++ values
+    // (-> meta_off).  vlscan_host_blocks_compress lays out its copied part with this same function, so that its buffer goes out as one DMA.
+    void put_headers(const vlscan_column& c, uint64_t bloom_len, DevColumn& d) {
+        if (c.kind == VLSCAN_COL_CONST) { d.meta_off = put(c.const_value, c.const_len); return; }
+        d.bloom_off = put(c.bloom, bloom_len);
+        if (c.value_type != VT_DICT) return;
+        const uint32_t total = c.dict_len ? c.dict_offsets[c.dict_len] : 0;
+        if (c.dict_len && c.dict_blob == (const uint8_t*)c.dict_offsets + 4 * (c.dict_len + 1)) {
+            d.meta_off = put((const uint8_t*)c.dict_offsets, 4 * (c.dict_len + 1) + total);   // caller memory already has the device layout
+            return;
+        }
+        auto meta = std::make_unique<std::vector<uint8_t>>(4 * (c.dict_len + 1) + total);   // zeros: an empty dict has offsets[0] = 0
+        if (c.dict_len) memcpy(meta->data(), c.dict_offsets, 4 * (c.dict_len + 1));
+        if (total) memcpy(meta->data() + 4 * (c.dict_len + 1), c.dict_blob, total);
+        d.meta_off = put(meta->data(), meta->size());
+        owned.push_back(std::move(meta));
+    }
+};
+
+// What one upload puts where, decided on the host alone (no CUDA call): the column and timestamps tables, validated on the way (the
+// vlscan_block descriptors are untrusted input), the host pieces of the arena and of the compressed staging buffer, and the arena regions
+// the device decoder regenerates on-disk payloads into.
+//
+// `headers` places what the header dispatch and the bloom probes look at: column kinds, const values, bloom filters, dict tables.  `values`
+// places the timestamps and the values payloads.  Both make a full upload.  Headers alone leave every values payload on the host
+// (VALUES_DEFERRED); values alone continue the table of such a header phase with the values of the columns `need` marks and flag the
+// others VALUES_ABSENT.  On-disk values blocks are not copied into the arena: their bytes go to the compressed staging buffer as they are
+// and the device regenerates them (vl_zstd.cuh) into arena regions placed behind everything that is copied, so that host memory laid out
+// like the copied part still goes out as one DMA.
+class UploadPlan {
+public:
+    std::vector<DevColumn>& cols;     // [nblocks * nfields]
+    std::vector<DevTimestamps> tsv;   // [nblocks], or empty when no block came with its timestamps column
+    std::vector<uint32_t> rows;
+    ArenaLayout layout;               // the copied part of the arena
+    std::vector<Piece> zpieces;       // host -> compressed staging buffer: the on-disk values blocks, then the ZSTD timestamps blocks
+    uint64_t zbytes = 0;              // end of the last one
+    ZstdJob zjob;                     // the frames inside zpieces, with their arena destinations
+    std::vector<OndiskCol> ocols;     // lens header checks + lens_type / lens_const / data_const: k_finish_ondisk_cols
+    bool decode = false;              // the device decoder regenerates something
+    uint64_t arena_bytes = 0;
+
+    // need_bloom (may be NULL = all): per batch field, whether the program that will scan this batch ever probes that field's bloom filters.
+    // A filter nobody probes stays on the host (the reference reads a column's bloom filter lazily, only when a filter asks for it:
+    // getBloomFilterForColumn, block_search.go:411-439); the column is staged with an empty filter, which no kernel touches.
+    UploadPlan(const vlscan_block* blocks, uint64_t nblocks, uint32_t nfields, bool headers, bool values, const std::vector<char>* need_bloom,
+               const uint8_t* need, std::vector<DevColumn>& cols)
+        : cols(cols), blocks(blocks), nblocks(nblocks), nfields(nfields), headers(headers), values(values), need_bloom(need_bloom), need(need) {
+        if (nblocks > 0xFFFFFFF0ull) throw BadInput("too many blocks in one batch");
+        const size_t ncells = (size_t)nblocks * std::max<uint32_t>(nfields, 1);
+        if (headers) { cols.assign(ncells, DevColumn{}); memset(cols.data(), 0, cols.size() * sizeof(DevColumn)); }
+        else if (cols.size() != ncells || !need) throw BadInput("internal: values phase of a bloom-first upload without its header phase");
+        rows.resize(nblocks);
+    }
+
+    // The compressed pieces and their places in the staging buffer (values only).  They are known before anything else, so that the
+    // caller can have the DMA engine busy while the host walks frame and block headers.
+    void collect_compressed() {
+        uint64_t zc = collect_values_blocks(blocks, nblocks, zv, headers ? nullptr : need, nfields);
+        for (const ZValuesBlock& v : zv) if (v.n) zpieces.push_back({v.p, v.n, v.zoff});
+        // ZSTD-compressed timestamps blocks (marshal types 1 and 4) travel the same way, behind the values blocks
+        for (uint64_t b = 0; b < nblocks; b++) {
+            const vlscan_block& blk = blocks[b];
+            if (blk.ts_marshal_type != MT_ZSTD_NEAREST_DELTA2 && blk.ts_marshal_type != MT_ZSTD_NEAREST_DELTA) continue;
+            if (blk.timestamps_len > vl::part::kMaxTimestampsBlockSize) throw BadInput("timestamps block size cannot exceed 8 MiB");   // getTimestamps block_search.go:490-493
+            zts_off.push_back(zc);
+            if (blk.timestamps_len) zpieces.push_back({blk.timestamps, blk.timestamps_len, zc});
+            zc += blk.timestamps_len;
+        }
+        zbytes = zc;
+    }
+    // frame, block and section headers of the on-disk values blocks, on several host threads; a malformed block is reported when describe()
+    // gets to it
+    void walk_headers() {
+        zinfo.resize(zv.size());
+        if (!zv.empty()) zjob.add_values_blocks(zv.data(), zv.size(), host_threads(), zinfo.data(), &zbad, &zmsg);
+    }
+    size_t values_blocks() const { return zv.size(); }
+    // The descriptor pass: every block, its timestamps, its columns in the caller's order (the order of the arena pieces), then the
+    // regenerated regions behind the copied part.
+    void describe() {
+        for (uint64_t b = 0; b < nblocks; b++) {
+            const vlscan_block& blk = blocks[b];
+            if (blk.rows > (8u << 20)) throw BadInput("block rows exceed maxRowsPerBlock (8Mi)");   // consts.go:24
+            rows[b] = (uint32_t)blk.rows;
+            if (blk.ts_marshal_type && values) place_timestamps(b, blk);
+            for (uint32_t k = 0; k < blk.ncols; k++) {
+                const vlscan_column& c = blk.cols[k];
+                if (c.field >= nfields) throw BadInput("column refers to a field outside the batch field table");
+                place_column(b, blk, c, cols[(size_t)b * nfields + c.field]);
+            }
+        }
+        const uint64_t regen_base = (layout.cursor + kArenaAlign - 1) / kArenaAlign * kArenaAlign;
+        for (const Ondisk& o : ondisk) {
+            DevColumn& d = cols[o.col];
+            d.lens_off += regen_base; d.data_off += regen_base;
+            zjob.set_dst(o.lens_frame, regen_base + o.lens_rel); zjob.set_dst(o.data_frame, regen_base + o.data_rel);
+        }
+        for (const TsFrame& tf : ts_frames) { tsv[tf.block].off = regen_base + tf.rel; zjob.set_dst(tf.frame, regen_base + tf.rel); }
+        decode = !ondisk.empty() || !ts_frames.empty();
+        arena_bytes = (decode ? regen_base + regen_cursor : layout.cursor) + kArenaPad;
+    }
+
+private:
+    const vlscan_block* blocks; uint64_t nblocks; uint32_t nfields;
+    bool headers, values;
+    const std::vector<char>* need_bloom;
+    const uint8_t* need;
+    std::vector<ZValuesBlock> zv; std::vector<ZValuesInfo> zinfo; size_t zbad = SIZE_MAX, zo = 0; std::string zmsg;
+    std::vector<uint64_t> zts_off; size_t zt = 0;   // staging offsets of the ZSTD timestamps blocks
+    uint64_t regen_cursor = 0;                      // regenerated regions, relative to the end of the copied part until describe() has sized it
     struct Ondisk { uint64_t col; uint32_t lens_frame, data_frame; uint64_t lens_rel, data_rel; };
     std::vector<Ondisk> ondisk;
-    std::vector<OndiskCol> ocols;
-    // copy pieces: runs that are contiguous on both sides (src stride == dst stride) and live in pinned host memory go out as one
-    // cudaMemcpyAsync; everything else is packed through a pinned staging ring.
-    uint64_t h2d = 0;
-    const size_t CH = 64u << 20;
-    uint8_t* stage = nullptr; cudaEvent_t evs[2] = {nullptr, nullptr}; int cur = 0; size_t fill = 0; uint64_t chunk_dst = 0; bool chunk_open = false;
-    uint8_t* dev_base = nullptr;   // destination buffer of the pieces being copied
-    // All host->device payload copies run on the ctx's copy stream; the compute stream picks them up through events.  While the
-    // compressed staging buffer is being filled, `zmarks` records (end offset, event) pairs so that the decoder of a launch group can
-    // start as soon as the bytes of that group have landed, while later bytes are still in flight.
-    cudaStream_t cs = ctx->copy_stream;
-    // every event of this upload lives in `events`: destroyed when the function is left, by return or by exception (a worker that keeps
-    // hitting malformed parts must not leak one event per batch)
-    struct EventBag {
-        std::vector<cudaEvent_t> all;
-        cudaEvent_t make() { cudaEvent_t e; VL_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); all.push_back(e); return e; }
-        ~EventBag() { for (cudaEvent_t e : all) cudaEventDestroy(e); }
-    } events;
+    struct TsFrame { uint64_t block; uint32_t frame; uint64_t rel; };
+    std::vector<TsFrame> ts_frames;
+
+    // the timestamps column: encoded deltas as stored + timestampsHeader (block_header.go:990-997)
+    void place_timestamps(uint64_t b, const vlscan_block& blk) {
+        if (blk.ts_marshal_type > MT_NEAREST_DELTA) throw BadInput("unknown MarshalType of a timestamps block");
+        if (blk.timestamps_len > vl::part::kMaxTimestampsBlockSize) throw BadInput("timestamps block size cannot exceed 8 MiB");
+        if (tsv.empty()) { tsv.resize(nblocks); memset(tsv.data(), 0, nblocks * sizeof(DevTimestamps)); }
+        DevTimestamps& t = tsv[b];
+        t.first = blk.min_timestamp; t.max = blk.max_timestamp;
+        if (blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA2 || blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA) {
+            uint64_t regen = 0; uint32_t id = 0;
+            zjob.add_frame(blk.timestamps, blk.timestamps_len, zts_off[zt++], &regen, &id);   // throws on a malformed frame header
+            if (regen > 10ull * blk.rows + 16) throw BadInput("cannot unmarshal timestamps: the decompressed block is larger than its varints can be");
+            t.mt = blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA2 ? MT_NEAREST_DELTA2 : MT_NEAREST_DELTA;
+            t.len = (uint32_t)regen;
+            ts_frames.push_back({b, id, arena_reserve(regen_cursor, regen)});
+        } else {
+            t.mt = (uint8_t)blk.ts_marshal_type; t.len = (uint32_t)blk.timestamps_len;
+            t.off = layout.put(blk.timestamps, blk.timestamps_len);
+        }
+    }
+    // one column of one block, headers and / or values
+    void place_column(uint64_t b, const vlscan_block& blk, const vlscan_column& c, DevColumn& d) {
+        if (!headers) {   // the headers are on the device since the header phase; now the values of the columns the probe pass marked
+            if (c.kind != VLSCAN_COL_VALUES) return;
+            if (!need[b * nfields + c.field]) { d.values_state = VALUES_ABSENT; return; }
+            d.values_state = VALUES_STAGED;
+            place_values(b, blk, c, d);
+            return;
+        }
+        if (d.kind != COL_MISSING) throw BadInput("duplicate column for one field in a block");
+        if (c.kind == VLSCAN_COL_CONST) {
+            d.kind = COL_CONST; d.meta_len = (uint32_t)c.const_len;
+            layout.put_headers(c, 0, d);
+            return;
+        }
+        if (c.kind != VLSCAN_COL_VALUES) throw BadInput("unknown column kind");
+        if (c.value_type < VT_STRING || c.value_type >= VT_MAX) throw BadInput("unknown valueType");
+        d.kind = COL_VALUES; d.vt = c.value_type; d.min_value = c.min_value; d.max_value = c.max_value;
+        if (values) place_values(b, blk, c, d);
+        else {
+            if (c.stage != VLSCAN_STAGE_ONDISK && c.stage != VLSCAN_STAGE_DECODED) throw BadInput("unknown values stage");
+            d.values_state = VALUES_DEFERRED;
+        }
+        if (c.bloom_len % 8) throw BadInput("cannot unmarshal bloomFilter from src with size not multiple by 8");   // bloomfilter.go:59-61
+        const bool keep_bloom = !need_bloom || (*need_bloom)[c.field];
+        d.bloom_words = keep_bloom ? (uint32_t)(c.bloom_len / 8) : 0;
+        if (c.value_type == VT_DICT) {
+            if (c.dict_len > 8) throw BadInput("valuesDict may contain max 8 items");
+            d.dict_len = c.dict_len;
+            d.meta_len = c.dict_len ? c.dict_offsets[c.dict_len] : 0;
+        }
+        layout.put_headers(c, keep_bloom ? c.bloom_len : 0, d);
+    }
+    // the values payload of one column: on-disk stage -> regenerated by the device decoder, decoded stage -> copied
+    void place_values(uint64_t b, const vlscan_block& blk, const vlscan_column& c, DevColumn& d) {
+        if (c.stage == VLSCAN_STAGE_ONDISK) {
+            // stringsBlockUnmarshaler.unmarshal: bytesBlock(lens) ++ bytesBlock(data) (encoding.go:83-108).  The host reads the
+            // containers, the frame header and the block headers; the payload is regenerated on the device.
+            if (zo == zbad) throw BadInput(zmsg);
+            const uint64_t lens_len = zinfo[zo].lens_len, data_len = zinfo[zo].data_len;
+            const uint32_t f1 = (uint32_t)(2 * zo), f2 = f1 + 1;
+            zo++;
+            if (data_len > 0xFFFFFFFFull) throw BadInput("values block too large");
+            // the uint block type byte lands on offset 15 of its region, so the lens items behind it are 16-byte aligned
+            const uint64_t lr = arena_reserve(regen_cursor, lens_len + 15), dr = arena_reserve(regen_cursor, data_len);
+            d.lens_off = lr + 16; d.data_off = dr; d.data_len = data_len;
+            const uint64_t ci = (uint64_t)b * nfields + c.field;
+            ondisk.push_back({ci, f1, f2, lr + 15, dr});
+            ocols.push_back({ci, lens_len, blk.rows});
+        } else if (c.stage == VLSCAN_STAGE_DECODED) {
+            const uint8_t* lens_items = c.lens_items; const uint64_t lens_len = c.lens_items_len, data_len = c.data_len;
+            // unmarshalUint64Items header checks (encoding.go:246-336)
+            if (lens_len < 1) throw BadInput("cannot unmarshal uint64 block type from empty src");
+            uint8_t lt = lens_items[0];
+            if (lt > 7) throw BadInput("unexpected uint64 block type");
+            uint64_t want = lt < 4 ? (blk.rows << lt) : (1ull << (lt - 4));
+            if (lens_len - 1 != want) throw BadInput("unexpected block length for uint items");
+            d.lens_type = lt;
+            if (lt >= 4) { uint64_t v = 0; for (uint64_t i = 0; i < want; i++) v = (v << 8) | lens_items[1 + i]; if (v > 0xFFFFFFFFull) throw BadInput("row length does not fit 32 bits"); d.lens_const = (uint32_t)v; }
+            if (data_len > 0xFFFFFFFFull) throw BadInput("values block too large");
+            d.lens_off = layout.put(lens_items + 1, lens_len - 1);
+            d.data_off = layout.put(c.data, data_len); d.data_len = data_len;
+            // decode rule of encoding.go:113-120: rows >= 2, all lens equal, len(data) == lens[0] => every row = data
+            d.data_const = (blk.rows >= 2 && lt >= 4 && data_len == d.lens_const) ? 1 : 0;
+        } else throw BadInput("unknown values stage");
+    }
+};
+
+// cuPointerGetAttribute of the driver library the runtime has loaded (the runtime API only classifies single addresses)
+typedef int (*PointerAttrFn)(void*, int, unsigned long long);
+PointerAttrFn pointer_attr_fn() {
+    static const PointerAttrFn fn = [] { void* h = dlopen("libcuda.so.1", RTLD_NOW | RTLD_GLOBAL); return h ? (PointerAttrFn)dlsym(h, "cuPointerGetAttribute") : (PointerAttrFn) nullptr; }();
+    if (!fn) throw CudaFail("cuPointerGetAttribute not found in libcuda.so.1: page-locked host ranges cannot be told apart", (int)cudaErrorSharedObjectSymbolNotFound);
+    return fn;
+}
+
+// The host -> device payload copies of one upload, all on the ctx's copy stream; the compute stream picks them up through events.  A run of
+// pieces that are contiguous on both sides (src stride == dst stride) and lie inside one page-locked allocation goes out as one
+// cudaMemcpyAsync; everything else is packed into a pinned two-chunk staging ring.  Marked copies record (end offset, event) pairs, so
+// that the decoder of a launch group can start as soon as the bytes of that group have landed, while later bytes are still in flight.
+// Every event lives until the copier is destroyed, by return or by exception (a worker that keeps hitting malformed parts must not leak one
+// event per batch).
+class H2DCopier {
+public:
+    uint64_t h2d = 0;       // bytes this upload sent
+    bool staged = false;    // some run went through the staging ring
+
+    explicit H2DCopier(vlscan_ctx* ctx) : ctx(ctx), cs(ctx->copy_stream), pointer_attr(pointer_attr_fn()) {}
+    ~H2DCopier() { for (cudaEvent_t e : events) cudaEventDestroy(e); }
+    H2DCopier(const H2DCopier&) = delete;
+    H2DCopier& operator=(const H2DCopier&) = delete;
+
+    // Is [p, p + len) inside ONE page-locked allocation?  The driver knows the range of the allocation an address belongs to
+    // (RANGE_START_ADDR / RANGE_SIZE).  Pointer queries cost microseconds each and a part's descriptors come as tens of thousands of small
+    // pieces (timestamps, const values) out of the same mmap()ed files: the last answers are remembered.  A 2 MiB-aligned region around a
+    // pageable address is taken as pageable as a whole (if a page-locked allocation begins inside it, its pieces merely take the staging
+    // ring), a page-locked allocation by its exact range.
+    bool pinned(const uint8_t* p, uint64_t len) {
+        const uintptr_t a = (uintptr_t)p;
+        if (a >= pageable_lo && a < pageable_hi) return false;
+        if (a >= locked_lo && a + len <= locked_hi) return true;
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
+        if (at.type != cudaMemoryTypeHost) { pageable_lo = a & ~(uintptr_t)((2u << 20) - 1); pageable_hi = pageable_lo + (2u << 20); return false; }
+        unsigned long long base = 0; size_t size = 0;
+        if (pointer_attr(&base, 11 /* CU_POINTER_ATTRIBUTE_RANGE_START_ADDR */, (unsigned long long)a) != 0 ||
+            pointer_attr(&size, 12 /* CU_POINTER_ATTRIBUTE_RANGE_SIZE */, (unsigned long long)a) != 0) return false;
+        if (size) { locked_lo = (uintptr_t)base; locked_hi = (uintptr_t)(base + size); }
+        return (unsigned long long)a >= base && (unsigned long long)a + len <= base + size;
+    }
+    // pieces [i0, i1) to the device buffer `base`; with `marks`, every DMA records its end offset for wait_for.  The staging ring is
+    // flushed at the end.
+    void copy(const std::vector<Piece>& pieces, size_t i0, size_t i1, uint8_t* base, bool marks) {
+        dev_base = base; marking = marks;
+        size_t i = i0;
+        const size_t end = std::min(i1, pieces.size());
+        while (i < end) {
+            // maximal run of pieces laid out identically on both sides (same stride between source and destination)
+            size_t j = i;
+            while (j + 1 < end && pieces[j + 1].src > pieces[j].src && pieces[j + 1].src - pieces[i].src == (ptrdiff_t)(pieces[j + 1].dst - pieces[i].dst)) j++;
+            // one DMA for the whole run (gaps included) only when the run lies inside a single page-locked allocation: two pinned buffers
+            // that merely line up could have pageable memory between them
+            if (pinned(pieces[i].src, (pieces[j].dst - pieces[i].dst) + pieces[j].len)) {
+                flush();
+                // (split at piece boundaries every ~128 MB so that consumers can be released chunk by chunk)
+                size_t a = i;
+                while (a <= j) {
+                    size_t b2 = a;
+                    while (b2 < j && (pieces[b2].dst + pieces[b2].len) - pieces[a].dst < (128ull << 20)) b2++;
+                    const uint64_t len = (pieces[b2].dst - pieces[a].dst) + pieces[b2].len;
+                    VL_CUDA(cudaMemcpyAsync(dev_base + pieces[a].dst, pieces[a].src, len, cudaMemcpyHostToDevice, cs));
+                    if (marking) mark(pieces[b2].dst + pieces[b2].len);
+                    h2d += len; a = b2 + 1;
+                }
+                i = j + 1;
+                continue;
+            }
+            staged = true;
+            need_stage();
+            for (; i <= j; i++) {
+                const Piece& pc = pieces[i];
+                uint64_t done = 0;
+                while (done < pc.len) {
+                    if (chunk_open && (chunk_dst + fill != pc.dst + done || fill == CH)) flush();
+                    if (!chunk_open) { chunk_open = true; chunk_dst = pc.dst + done; fill = 0; }
+                    size_t take = (size_t)std::min<uint64_t>(pc.len - done, CH - fill);
+                    segs.push_back({pc.src + done, fill, take});
+                    fill += take; done += take;
+                }
+                // pack the space up to the next piece as zeros when it follows closely, so chunks stay large: between two pieces of the copied
+                // part there is nothing but alignment slack and empty reservations (a bloom filter left on the host is 48 bytes of them), zero
+                // in the arena already.  With a 64-byte limit every timestamps block of a part was a chunk, a DMA and an event of its own: 16 k
+                // per batch.
+                if (i + 1 < end) {
+                    uint64_t gap = pieces[i + 1].dst - (pc.dst + pc.len);
+                    if (gap <= 1024 && fill + gap < CH) { if (gap) segs.push_back({nullptr, fill, (size_t)gap}); fill += gap; } else flush();
+                }
+            }
+        }
+        flush();
+    }
+    // The compressed staging buffer is filled in order: enqueue every piece of `z` not sent yet that starts below `limit`, marked
+    void copy_compressed(const std::vector<Piece>& z, uint8_t* zsrc, uint64_t limit) {
+        size_t hi = zsent;
+        while (hi < z.size() && z[hi].dst < limit) hi++;
+        if (hi == zsent) return;
+        copy(z, zsent, hi, zsrc, true);
+        zsent = hi;
+    }
+    // `st` waits until the marked copies have landed up to source offset `src_end`
+    void wait_for(cudaStream_t st, uint64_t src_end) {
+        for (auto& m : zmarks) if (m.first >= src_end) { VL_CUDA(cudaStreamWaitEvent(st, m.second, 0)); return; }
+        if (!zmarks.empty()) VL_CUDA(cudaStreamWaitEvent(st, zmarks.back().second, 0));
+    }
+    // a table built on the host, counted like the pieces
+    void copy_table(void* dst, const void* src, size_t n) { if (n) VL_CUDA(cudaMemcpyAsync(dst, src, n, cudaMemcpyHostToDevice, cs)); h2d += n; }
+    // the copies enqueued from now on start after what `st` has enqueued so far
+    void after(cudaStream_t st) { cudaEvent_t e = make(); VL_CUDA(cudaEventRecord(e, st)); VL_CUDA(cudaStreamWaitEvent(cs, e, 0)); }
+    // an event that completes with every copy enqueued so far
+    cudaEvent_t done() { cudaEvent_t e = make(); VL_CUDA(cudaEventRecord(e, cs)); return e; }
+
+private:
+    static constexpr size_t CH = 64u << 20;   // staging ring chunk
+    vlscan_ctx* ctx; cudaStream_t cs;
+    PointerAttrFn pointer_attr;
+    std::vector<cudaEvent_t> events;
     std::vector<std::pair<uint64_t, cudaEvent_t>> zmarks;
-    bool marking = false;
-    auto mark = [&](uint64_t end_off) { cudaEvent_t e = events.make(); VL_CUDA(cudaEventRecord(e, cs)); zmarks.push_back({end_off, e}); };
+    size_t zsent = 0;
+    uintptr_t pageable_lo = 1, pageable_hi = 0, locked_lo = 1, locked_hi = 0;
+    // the ring, and the copy being made
+    uint8_t* stage = nullptr; cudaEvent_t evs[2] = {nullptr, nullptr}; int cur = 0; size_t fill = 0; uint64_t chunk_dst = 0; bool chunk_open = false;
+    uint8_t* dev_base = nullptr; bool marking = false;
     // Packing pageable memory (a part's mmap()ed files) into the ring is a memcpy, ~10 GB/s on one core and page faults on cold files: the
-    // segments of a chunk are only recorded while the pieces are walked, and copied by all host threads when the chunk is flushed
-    // (each thread takes an equal byte range of the chunk).
+    // segments of a chunk are only recorded while the pieces are walked, and copied by all host threads when the chunk is flushed (each
+    // thread takes an equal byte range of the chunk).
     struct Seg { const uint8_t* src; size_t at, len; };   // src == nullptr: zeros
     std::vector<Seg> segs;
-    auto pack_chunk = [&](uint8_t* buf, size_t bytes) {
+
+    cudaEvent_t make() { cudaEvent_t e; VL_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); events.push_back(e); return e; }
+    void mark(uint64_t end_off) { cudaEvent_t e = make(); VL_CUDA(cudaEventRecord(e, cs)); zmarks.push_back({end_off, e}); }
+    void need_stage() {
+        if (stage) return;
+        stage = (uint8_t*)ctx->ensure_pinned(2 * CH);
+        for (int k = 0; k < 2; k++) { evs[k] = make(); VL_CUDA(cudaEventRecord(evs[k], cs)); }
+    }
+    void pack_chunk(uint8_t* buf, size_t bytes) {
         const int nt = (int)std::min<size_t>(std::max(1, host_threads()), bytes / (1u << 20) + 1);
         auto work = [&](int t) {
             const size_t lo = bytes * (size_t)t / nt, hi = bytes * (size_t)(t + 1) / nt;
@@ -239,8 +525,8 @@ static void do_upload(vlscan_ctx* ctx, const char* const* field_names, const siz
         if (nt <= 1) { work(0); return; }
         if (!ctx->pool) ctx->pool = new HostPool;
         ctx->pool->run(nt, work);
-    };
-    auto flush = [&]() {
+    }
+    void flush() {
         if (!chunk_open || !fill) { chunk_open = false; fill = 0; segs.clear(); return; }
         pack_chunk(stage + (size_t)cur * CH, fill);
         segs.clear();
@@ -249,283 +535,93 @@ static void do_upload(vlscan_ctx* ctx, const char* const* field_names, const siz
         if (marking) mark(chunk_dst + fill);
         h2d += fill; cur ^= 1; fill = 0; chunk_open = false;
         VL_CUDA(cudaEventSynchronize(evs[cur]));
-    };
-    auto is_pinned = [&](const void* p) { cudaPointerAttributes a; if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; } return a.type == cudaMemoryTypeHost; };
-    // Is [p, p + len) inside ONE page-locked allocation?  The runtime API only classifies single addresses; the driver knows the range of the
-    // allocation an address belongs to (cuPointerGetAttribute RANGE_START_ADDR / RANGE_SIZE).  libcuda is always there when a device is.
-    // Pointer queries cost microseconds each and a part's descriptors come as tens of thousands of small pieces (timestamps, const values) out of
-    // the same mmap()ed files: the last answers are remembered.  A 2 MiB-aligned region around a pageable address is taken as pageable as a whole
-    // (if a page-locked allocation begins inside it, its pieces merely take the staging ring), a page-locked allocation by its exact range.
-    uintptr_t pageable_lo = 1, pageable_hi = 0, locked_lo = 1, locked_hi = 0;
-    auto pinned_range_covers = [&](const uint8_t* p, uint64_t len) -> bool {
-        typedef int (*attr_fn)(void*, int, unsigned long long);
-        static const attr_fn fn = [] { void* h = dlopen("libcuda.so.1", RTLD_NOW | RTLD_GLOBAL); return h ? (attr_fn)dlsym(h, "cuPointerGetAttribute") : (attr_fn) nullptr; }();
-        const uintptr_t a = (uintptr_t)p;
-        if (a >= pageable_lo && a < pageable_hi) return false;
-        if (a >= locked_lo && a + len <= locked_hi) return true;
-        if (!is_pinned(p)) { pageable_lo = a & ~(uintptr_t)((2u << 20) - 1); pageable_hi = pageable_lo + (2u << 20); return false; }
-        if (!fn) return len <= 1 || (len <= 4096 && is_pinned(p + len - 1));   // no driver entry point: only what single-address checks can vouch for
-        unsigned long long base = 0; size_t size = 0;
-        if (fn(&base, 11 /* CU_POINTER_ATTRIBUTE_RANGE_START_ADDR */, (unsigned long long)(uintptr_t)p) != 0 || fn(&size, 12 /* CU_POINTER_ATTRIBUTE_RANGE_SIZE */, (unsigned long long)(uintptr_t)p) != 0) return false;
-        if (size) { locked_lo = (uintptr_t)base; locked_hi = (uintptr_t)(base + size); }
-        return (unsigned long long)(uintptr_t)p >= base && (unsigned long long)(uintptr_t)p + len <= base + size;
-    };
-    auto need_stage = [&]() {
-        if (stage) return;
-        stage = (uint8_t*)ctx->ensure_pinned(2 * CH);
-        for (int k = 0; k < 2; k++) { evs[k] = events.make(); VL_CUDA(cudaEventRecord(evs[k], cs)); }
-    };
-    bool all_pinned = true;
-    // pieces [i0, i1) of the list (all of it by default); the staging ring is flushed at the end of every call
-    auto copy_pieces = [&](const std::vector<Piece>& pieces, uint8_t* base, size_t i0 = 0, size_t i1 = SIZE_MAX) {
-    dev_base = base;
-    size_t i = i0;
-    const size_t end = std::min(i1, pieces.size());
-    while (i < end) {
-        // maximal run of pieces laid out identically on both sides (same stride between source and destination)
-        size_t j = i;
-        while (j + 1 < end && pieces[j + 1].src > pieces[j].src && pieces[j + 1].src - pieces[i].src == (ptrdiff_t)(pieces[j + 1].dst - pieces[i].dst)) j++;
-        uint64_t run_len = (pieces[j].dst - pieces[i].dst) + pieces[j].len;
-        // one DMA for the whole run (gaps included) only when the run lies inside a single page-locked allocation: two pinned buffers that
-        // merely line up could have pageable memory between them
-        if (pinned_range_covers(pieces[i].src, run_len)) {
-            // page-locked caller memory: one DMA for the whole run, gaps (alignment slack) included
-            flush();
-            // (split at piece boundaries every ~128 MB so that consumers can be released chunk by chunk)
-            size_t a = i;
-            while (a <= j) {
-                size_t b2 = a;
-                while (b2 < j && (pieces[b2].dst + pieces[b2].len) - pieces[a].dst < (128ull << 20)) b2++;
-                const uint64_t len = (pieces[b2].dst - pieces[a].dst) + pieces[b2].len;
-                VL_CUDA(cudaMemcpyAsync(dev_base + pieces[a].dst, pieces[a].src, len, cudaMemcpyHostToDevice, cs));
-                if (marking) mark(pieces[b2].dst + pieces[b2].len);
-                h2d += len; a = b2 + 1;
-            }
-            (void)run_len;
-            i = j + 1;
-            continue;
-        }
-        all_pinned = false;
-        need_stage();
-        for (; i <= j; i++) {
-            const Piece& pc = pieces[i];
-            uint64_t done = 0;
-            while (done < pc.len) {
-                if (chunk_open && (chunk_dst + fill != pc.dst + done || fill == CH)) flush();
-                if (!chunk_open) { chunk_open = true; chunk_dst = pc.dst + done; fill = 0; }
-                size_t take = (size_t)std::min<uint64_t>(pc.len - done, CH - fill);
-                segs.push_back({pc.src + done, fill, take});
-                fill += take; done += take;
-            }
-            // pack the space up to the next piece as zeros when it follows closely, so chunks stay large: between two pieces of the copied part
-            // there is nothing but alignment slack and empty reservations (a bloom filter left on the host is 48 bytes of them), zero in the
-            // arena already.  With a 64-byte limit every timestamps block of a part was a chunk, a DMA and an event of its own: 16 k per batch.
-            if (i + 1 < end) {
-                uint64_t gap = pieces[i + 1].dst - (pc.dst + pc.len);
-                if (gap <= 1024 && fill + gap < CH) { if (gap) segs.push_back({nullptr, fill, (size_t)gap}); fill += gap; } else flush();
-            }
-        }
     }
-    flush();
-    };
-    // Pre-pass: the compressed bytes of on-disk values blocks are shipped first (their place in the staging buffer is a running sum), so
-    // that the DMA engine is busy while the host walks frame and block headers.
-    bool zlazy = false; size_t zcopied = 0;   // zpieces[0, zcopied) are on their way to the compressed staging buffer
-    auto advance_z = [&](uint64_t limit) {      // enqueue every compressed piece that starts below `limit`
-        size_t hi = zcopied;
-        while (hi < zpieces.size() && zpieces[hi].dst < limit) hi++;
-        if (hi == zcopied) return;
-        marking = true; copy_pieces(zpieces, ctx->zsrc.as<uint8_t>(), zcopied, hi); marking = false;
-        zcopied = hi;
-    };
-    std::vector<ZValuesBlock> zv, zts; std::vector<ZValuesInfo> zinfo; size_t zbad = SIZE_MAX, zo = 0, zt = 0; std::string zmsg;
-    std::vector<DevTimestamps> tsv; bool any_ts = false;
-    struct TsFrame { uint64_t block; uint32_t frame; uint64_t rel; };
-    std::vector<TsFrame> ts_frames;
-    if (mode != UP_HEADERS) {
-        uint64_t zc = collect_values_blocks(blocks, nblocks, zv, mode == UP_VALUES ? need : nullptr, nfields);
-        for (const ZValuesBlock& v : zv) if (v.n) zpieces.push_back({v.p, v.n, v.zoff});
-        // ZSTD-compressed timestamps blocks (marshal types 1 and 4) travel the same way, behind the values blocks
-        for (uint64_t b = 0; b < nblocks; b++) {
-            const vlscan_block& blk = blocks[b];
-            if (blk.ts_marshal_type != MT_ZSTD_NEAREST_DELTA2 && blk.ts_marshal_type != MT_ZSTD_NEAREST_DELTA) continue;
-            if (blk.timestamps_len > vl::part::kMaxTimestampsBlockSize) throw BadInput("timestamps block size cannot exceed 8 MiB");   // getTimestamps block_search.go:490-493
-            zts.push_back({blk.timestamps, (size_t)blk.timestamps_len, zc});
-            if (blk.timestamps_len) zpieces.push_back({blk.timestamps, blk.timestamps_len, zc});
-            zc += blk.timestamps_len;
+};
+}  // namespace
+
+// mode: UP_FULL stages everything in one go.  A bloom-first upload (vlscan_scan_batch, the reference's lazy order: a column's values are read only
+// after its bloom filter let the block through, block_search.go:411-439 then :444-474) runs the function twice around the probe pass:
+// UP_HEADERS stages the headers (-> batch->harena), UP_VALUES then the timestamps and the values of the columns the probe marked in `need`
+// (-> batch->arena).
+enum UploadMode { UP_FULL = 0, UP_HEADERS = 1, UP_VALUES = 2 };
+static void do_upload(vlscan_ctx* ctx, const char* const* field_names, const size_t* field_name_lens, uint32_t nfields, const vlscan_block* blocks,
+                      uint64_t nblocks, vlscan_batch* out, vlscan_stats* stats, const std::vector<char>* need_bloom = nullptr, UploadMode mode = UP_FULL,
+                      const uint8_t* need = nullptr) {
+    VL_CUDA(cudaSetDevice(ctx->device));
+    const bool dbg = getenv("VLSCAN_DEBUG_TIMING") != nullptr;
+    auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+    double t_start = now(), t_desc = 0, t_alloc = 0, t_copy = 0;
+    const bool headers = mode != UP_VALUES, values = mode != UP_HEADERS;
+    UploadPlan plan(blocks, nblocks, nfields, headers, values, need_bloom, need, out->h_cols);
+    out->device = ctx->device; out->nfields = nfields;
+    if (headers) for (uint32_t f = 0; f < nfields; f++) out->field_names.emplace_back(field_names[f], field_name_lens[f]);
+    out->split_hdr = !(headers && values);
+    DevBuf& arena = values ? out->arena : out->harena;
+    H2DCopier copier(ctx);
+    bool zlazy = false;
+    if (values) {
+        plan.collect_compressed();
+        // Page-locked sources: everything is enqueued right away (asynchronous DMA), so that the DMA engine is busy while the host walks the
+        // headers.  Pageable sources (a part's mmap()ed files) have to be packed through the staging ring by this thread: that is done lazily,
+        // launch group by launch group, from the decoder's group hook below, so that the device decodes group g while the host packs group
+        // g + 1 (packing it all here would finish before the first kernel starts).
+        if (!plan.zpieces.empty()) {
+            ctx->zsrc.ensure(plan.zbytes + 512);
+            zlazy = !copier.pinned(plan.zpieces[0].src, plan.zpieces[0].len);
+            if (!zlazy) copier.copy_compressed(plan.zpieces, ctx->zsrc.as<uint8_t>(), UINT64_MAX);
         }
-        // Page-locked sources: everything is enqueued right away (asynchronous DMA).  Pageable sources (a part's mmap()ed files) have to be packed
-        // through the staging ring by this thread: that is done lazily, launch group by launch group, from the decoder's group hook below, so
-        // that the device decodes group g while the host packs group g + 1 (packing it all here would finish before the first kernel starts).
-        if (!zpieces.empty()) { ctx->zsrc.ensure(zc + 512); zlazy = !pinned_range_covers(zpieces[0].src, zpieces[0].len); if (!zlazy) advance_z(UINT64_MAX); }
-        // frame, block and section headers of all of them, on several host threads; a malformed block is reported when the loop below gets to it
-        zinfo.resize(zv.size());
         const double t_w = now();
-        if (!zv.empty()) zjob.add_values_blocks(zv.data(), zv.size(), host_threads(), zinfo.data(), &zbad, &zmsg);
+        plan.walk_headers();
         if (dbg) fprintf(stderr, "[vlscan upload] header walk of %zu values blocks on %d host threads: %.1f ms (after %.1f ms of collecting and enqueueing the copies)\n",
-                         zv.size(), host_threads(), 1e3 * (now() - t_w), 1e3 * (t_w - t_start));
+                         plan.values_blocks(), host_threads(), 1e3 * (now() - t_w), 1e3 * (t_w - t_start));
     }
-    // the values payload of one column: on-disk stage -> regenerated by the device decoder, decoded stage -> copied
-    auto stage_values = [&](const vlscan_block& blk, const vlscan_column& c, DevColumn& d, uint64_t b) {
-            if (c.stage == VLSCAN_STAGE_ONDISK) {
-                // stringsBlockUnmarshaler.unmarshal: bytesBlock(lens) ++ bytesBlock(data) (encoding.go:83-108).  The host reads the
-                // containers, the frame header and the block headers; the payload is regenerated on the device.
-                if (zo == zbad) throw BadInput(zmsg);
-                const uint64_t lens_len = zinfo[zo].lens_len, data_len = zinfo[zo].data_len;
-                const uint32_t f1 = (uint32_t)(2 * zo), f2 = f1 + 1;
-                zo++;
-                if (data_len > 0xFFFFFFFFull) throw BadInput("values block too large");
-                // the uint block type byte lands on offset 15 of its region, so the lens items behind it are 16-byte aligned
-                const uint64_t lr = arena_reserve(regen_cursor, lens_len + 15), dr = arena_reserve(regen_cursor, data_len);
-                d.lens_off = lr + 16; d.data_off = dr; d.data_len = data_len;
-                const uint64_t ci = (uint64_t)b * nfields + c.field;
-                ondisk.push_back({ci, f1, f2, lr + 15, dr});
-                ocols.push_back({ci, lens_len, blk.rows});   // lens header checks + lens_type / lens_const / data_const: k_finish_ondisk_cols
-            } else if (c.stage == VLSCAN_STAGE_DECODED) {
-                const uint8_t* lens_items = c.lens_items; const uint64_t lens_len = c.lens_items_len, data_len = c.data_len;
-                // unmarshalUint64Items header checks (encoding.go:246-336)
-                if (lens_len < 1) throw BadInput("cannot unmarshal uint64 block type from empty src");
-                uint8_t lt = lens_items[0];
-                if (lt > 7) throw BadInput("unexpected uint64 block type");
-                uint64_t want = lt < 4 ? (blk.rows << lt) : (1ull << (lt - 4));
-                if (lens_len - 1 != want) throw BadInput("unexpected block length for uint items");
-                d.lens_type = lt;
-                if (lt >= 4) { uint64_t v = 0; for (uint64_t i = 0; i < want; i++) v = (v << 8) | lens_items[1 + i]; if (v > 0xFFFFFFFFull) throw BadInput("row length does not fit 32 bits"); d.lens_const = (uint32_t)v; }
-                if (data_len > 0xFFFFFFFFull) throw BadInput("values block too large");
-                d.lens_off = add_piece(lens_items + 1, lens_len - 1);
-                d.data_off = add_piece(c.data, data_len); d.data_len = data_len;
-                // decode rule of encoding.go:113-120: rows >= 2, all lens equal, len(data) == lens[0] => every row = data
-                d.data_const = (blk.rows >= 2 && lt >= 4 && data_len == d.lens_const) ? 1 : 0;
-            } else throw BadInput("unknown values stage");
-    };
-    for (uint64_t b = 0; b < nblocks; b++) {
-        const vlscan_block& blk = blocks[b];
-        if (blk.rows > (8u << 20)) throw BadInput("block rows exceed maxRowsPerBlock (8Mi)");   // consts.go:24
-        rows[b] = (uint32_t)blk.rows;
-        if (blk.ts_marshal_type && mode != UP_HEADERS) {   // the timestamps column: encoded deltas as stored + timestampsHeader (block_header.go:990-997)
-            if (blk.ts_marshal_type > MT_NEAREST_DELTA) throw BadInput("unknown MarshalType of a timestamps block");
-            if (blk.timestamps_len > vl::part::kMaxTimestampsBlockSize) throw BadInput("timestamps block size cannot exceed 8 MiB");
-            if (tsv.empty()) { tsv.resize(nblocks); memset(tsv.data(), 0, nblocks * sizeof(DevTimestamps)); }
-            any_ts = true;
-            DevTimestamps& t = tsv[b];
-            t.first = blk.min_timestamp; t.max = blk.max_timestamp;
-            if (blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA2 || blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA) {
-                uint64_t regen = 0; uint32_t id = 0;
-                zjob.add_frame(zts[zt].p, zts[zt].n, zts[zt].zoff, &regen, &id);   // throws on a malformed frame header
-                zt++;
-                if (regen > 10ull * blk.rows + 16) throw BadInput("cannot unmarshal timestamps: the decompressed block is larger than its varints can be");
-                t.mt = blk.ts_marshal_type == MT_ZSTD_NEAREST_DELTA2 ? MT_NEAREST_DELTA2 : MT_NEAREST_DELTA;
-                t.len = (uint32_t)regen;
-                ts_frames.push_back({b, id, arena_reserve(regen_cursor, regen)});
-            } else {
-                t.mt = (uint8_t)blk.ts_marshal_type; t.len = (uint32_t)blk.timestamps_len;
-                t.off = add_piece(blk.timestamps, blk.timestamps_len);
-            }
-        }
-        for (uint32_t k = 0; k < blk.ncols; k++) {
-            const vlscan_column& c = blk.cols[k];
-            if (c.field >= nfields) throw BadInput("column refers to a field outside the batch field table");
-            DevColumn& d = cols[(size_t)b * nfields + c.field];
-            if (mode == UP_VALUES) {   // the headers are on the device since phase 1; now the values of the columns the probe pass marked
-                if (c.kind != VLSCAN_COL_VALUES) continue;
-                if (!need[b * nfields + c.field]) { d.values_state = VALUES_ABSENT; continue; }
-                d.values_state = VALUES_STAGED;
-                stage_values(blk, c, d, b);
-                continue;
-            }
-            if (d.kind != COL_MISSING) throw BadInput("duplicate column for one field in a block");
-            if (c.kind == VLSCAN_COL_CONST) {
-                d.kind = COL_CONST; d.meta_len = (uint32_t)c.const_len; d.meta_off = add_piece(c.const_value, c.const_len);
-                continue;
-            }
-            if (c.kind != VLSCAN_COL_VALUES) throw BadInput("unknown column kind");
-            if (c.value_type < VT_STRING || c.value_type >= VT_MAX) throw BadInput("unknown valueType");
-            d.kind = COL_VALUES; d.vt = c.value_type; d.min_value = c.min_value; d.max_value = c.max_value;
-            if (mode == UP_HEADERS) {
-                if (c.stage != VLSCAN_STAGE_ONDISK && c.stage != VLSCAN_STAGE_DECODED) throw BadInput("unknown values stage");
-                d.values_state = VALUES_DEFERRED;
-            } else stage_values(blk, c, d, b);
-            if (c.bloom_len % 8) throw BadInput("cannot unmarshal bloomFilter from src with size not multiple by 8");   // bloomfilter.go:59-61
-            if (need_bloom && !(*need_bloom)[c.field]) { d.bloom_words = 0; d.bloom_off = add_piece(c.bloom, 0); }
-            else { d.bloom_words = (uint32_t)(c.bloom_len / 8); d.bloom_off = add_piece(c.bloom, c.bloom_len); }
-            if (c.value_type == VT_DICT) {
-                if (c.dict_len > 8) throw BadInput("valuesDict may contain max 8 items");
-                d.dict_len = c.dict_len;
-                uint32_t total = c.dict_len ? c.dict_offsets[c.dict_len] : 0;
-                d.meta_len = total;
-                if (c.dict_len && c.dict_blob == (const uint8_t*)c.dict_offsets + 4 * (c.dict_len + 1)) {
-                    d.meta_off = add_piece((const uint8_t*)c.dict_offsets, 4 * (c.dict_len + 1) + total);   // caller memory already has the device layout
-                } else {
-                    auto meta = std::make_unique<std::vector<uint8_t>>();
-                    meta->resize(4 * (c.dict_len + 1) + total);
-                    if (c.dict_len) memcpy(meta->data(), c.dict_offsets, 4 * (c.dict_len + 1)); else memset(meta->data(), 0, 4);
-                    if (total) memcpy(meta->data() + 4 * (c.dict_len + 1), c.dict_blob, total);
-                    d.meta_off = add_piece(meta->data(), meta->size());
-                    owned.push_back(std::move(meta));
-                }
-            }
-        }
-    }
-    // regenerated regions follow the copied part
-    const uint64_t regen_base = (cursor + kArenaAlign - 1) / kArenaAlign * kArenaAlign;
-    for (const Ondisk& o : ondisk) {
-        DevColumn& d = cols[o.col];
-        d.lens_off += regen_base; d.data_off += regen_base;
-        zjob.set_dst(o.lens_frame, regen_base + o.lens_rel); zjob.set_dst(o.data_frame, regen_base + o.data_rel);
-    }
-    for (const TsFrame& tf : ts_frames) { tsv[tf.block].off = regen_base + tf.rel; zjob.set_dst(tf.frame, regen_base + tf.rel); }
-    if (!ondisk.empty() || !ts_frames.empty()) cursor = regen_base + regen_cursor;
-    const uint64_t arena_bytes = cursor + kArenaPad;
-    (mode == UP_HEADERS ? out->harena_bytes : out->arena_bytes) = arena_bytes;
-    if (mode == UP_FULL) out->harena_bytes = 0;
+    plan.describe();
+    (values ? out->arena_bytes : out->harena_bytes) = plan.arena_bytes;
+    if (headers && values) out->harena_bytes = 0;
     t_desc = now();
-    arena_buf.ensure(arena_bytes);
+    arena.ensure(plan.arena_bytes);
     t_alloc = now();
     // the arena is cleared on the compute stream; the copy stream takes over from there
-    cudaEvent_t ev_cleared = events.make(), ev_copied = events.make();
-    VL_CUDA(cudaMemsetAsync(arena_buf.p, 0, arena_bytes, ctx->stream));
-    VL_CUDA(cudaEventRecord(ev_cleared, ctx->stream));
-    VL_CUDA(cudaStreamWaitEvent(cs, ev_cleared, 0));
+    VL_CUDA(cudaMemsetAsync(arena.p, 0, plan.arena_bytes, ctx->stream));
+    copier.after(ctx->stream);
     // The decoder is enqueued BEFORE anything below that can block this thread (packing pageable pieces through the staging ring, copies
     // from pageable vectors): each launch group then runs as soon as its compressed bytes have landed, beside the DMA of the later ones.
-    const bool have_z = !ondisk.empty() || !ts_frames.empty();
     double t_h2d = 0, t_zrun = 0;
     if (dbg) t_h2d = now();
-    if (have_z) {
-        zjob.set_group_hook([&](uint64_t src_end) {
-            if (zlazy) advance_z(src_end);
-            for (auto& m : zmarks) if (m.first >= src_end) { VL_CUDA(cudaStreamWaitEvent(ctx->stream, m.second, 0)); return; }
-            if (!zmarks.empty()) VL_CUDA(cudaStreamWaitEvent(ctx->stream, zmarks.back().second, 0));
+    if (plan.decode) {
+        plan.zjob.set_group_hook([&](uint64_t src_end) {
+            if (zlazy) copier.copy_compressed(plan.zpieces, ctx->zsrc.as<uint8_t>(), src_end);
+            copier.wait_for(ctx->stream, src_end);
         });
-        zjob.run(ctx, ctx->zsrc.as<uint8_t>(), arena_buf.as<uint8_t>());
-        if (zlazy) advance_z(UINT64_MAX);
+        plan.zjob.run(ctx, ctx->zsrc.as<uint8_t>(), arena.as<uint8_t>());
+        if (zlazy) copier.copy_compressed(plan.zpieces, ctx->zsrc.as<uint8_t>(), UINT64_MAX);
         if (dbg) t_zrun = now();
     }
-    copy_pieces(pieces, arena_buf.as<uint8_t>());
+    copier.copy(plan.layout.pieces, 0, plan.layout.pieces.size(), arena.as<uint8_t>(), false);
+    const std::vector<DevColumn>& cols = plan.cols;
     out->cols.ensure(std::max<size_t>(cols.size() * sizeof(DevColumn), 16));
-    if (!cols.empty()) VL_CUDA(cudaMemcpyAsync(out->cols.p, cols.data(), cols.size() * sizeof(DevColumn), cudaMemcpyHostToDevice, cs));
-    if (mode != UP_HEADERS) out->has_ts = any_ts; else out->has_ts = false;
-    if (any_ts) {
+    copier.copy_table(out->cols.p, cols.data(), cols.size() * sizeof(DevColumn));
+    out->has_ts = !plan.tsv.empty();
+    if (out->has_ts) {
         out->ts.ensure(nblocks * sizeof(DevTimestamps));
-        VL_CUDA(cudaMemcpyAsync(out->ts.p, tsv.data(), nblocks * sizeof(DevTimestamps), cudaMemcpyHostToDevice, cs));
-        h2d += nblocks * sizeof(DevTimestamps);
+        copier.copy_table(out->ts.p, plan.tsv.data(), nblocks * sizeof(DevTimestamps));
     }
-    VL_CUDA(cudaEventRecord(ev_copied, cs));
-    h2d += cols.size() * sizeof(DevColumn);
+    const cudaEvent_t ev_copied = copier.done();
     const double t_enq = dbg ? now() : 0;
-    if (have_z) {
+    if (plan.decode) {
         // the on-disk payloads are being regenerated in HBM; derive lens_type / lens_const / data_const from the regenerated lens blocks
+        const std::vector<OndiskCol>& ocols = plan.ocols;
         VL_CUDA(cudaStreamWaitEvent(ctx->stream, ev_copied, 0));
         ctx->zcols.ensure(16 + ocols.size() * sizeof(OndiskCol));
         VL_CUDA(cudaMemsetAsync(ctx->zcols.p, 0, 16, ctx->stream));
         VL_CUDA(cudaMemcpyAsync(ctx->zcols.as<uint8_t>() + 16, ocols.data(), ocols.size() * sizeof(OndiskCol), cudaMemcpyHostToDevice, ctx->stream));
         if (!ocols.empty()) {
-            k_finish_ondisk_cols<<<cdiv(ocols.size(), 128), 128, 0, ctx->stream>>>(arena_buf.as<uint8_t>(), out->cols.as<DevColumn>(), (const OndiskCol*)(ctx->zcols.as<uint8_t>() + 16),
+            k_finish_ondisk_cols<<<cdiv(ocols.size(), 128), 128, 0, ctx->stream>>>(arena.as<uint8_t>(), out->cols.as<DevColumn>(), (const OndiskCol*)(ctx->zcols.as<uint8_t>() + 16),
                                                                                      (uint32_t)ocols.size(), ctx->zcols.as<unsigned long long>());
             launch_check(ctx);
         }
-        h2d += ocols.size() * sizeof(OndiskCol);
-        zjob.check(ctx);   // synchronises the stream
+        copier.h2d += ocols.size() * sizeof(OndiskCol);
+        plan.zjob.check(ctx);   // synchronises the stream
         unsigned long long cst[2] = {0, 0};
         VL_CUDA(cudaMemcpy(cst, ctx->zcols.p, 16, cudaMemcpyDeviceToHost));
         static const char* what[] = {"", "cannot unmarshal uint64 block type from empty src", "unexpected uint64 block type", "unexpected block length for uint items", "row length does not fit 32 bits"};
@@ -534,15 +630,15 @@ static void do_upload(vlscan_ctx* ctx, const char* const* field_names, const siz
     VL_CUDA(cudaStreamWaitEvent(ctx->stream, ev_copied, 0));
     if (dbg) { VL_CUDA(cudaStreamSynchronize(ctx->stream)); t_copy = now(); }
     if (nfields) out->note_columns(cols);
-    if (mode != UP_VALUES) finish_batch_layout(ctx, out, rows);   // synchronises the stream => `owned`, `cols`, staging are safe to drop
-    else VL_CUDA(cudaStreamSynchronize(ctx->stream));             // the layout tables are there since the header phase
+    if (headers) finish_batch_layout(ctx, out, plan.rows);   // synchronises the stream => the plan's tables and the staging ring are free again
+    else VL_CUDA(cudaStreamSynchronize(ctx->stream));        // the layout tables are there since the header phase
+    uint64_t h2d = copier.h2d;
     if (dbg) fprintf(stderr, "[vlscan upload] blocks=%llu arena=%.1f MB h2d=%.1f MB pieces=%zu+%zu pinned=%d: describe %.1f ms, alloc %.1f ms, copy %.1f ms (%.1f GB/s), "
                              "zstd %llu frames / %llu blocks / %llu sequences: enqueue %.1f ms, decode %.1f ms; layout %.1f ms\n", (unsigned long long)nblocks,
-                     arena_bytes / 1e6, h2d / 1e6, pieces.size(), zpieces.size(), (int)all_pinned, 1e3 * (t_desc - t_start), 1e3 * (t_alloc - t_desc), 1e3 * (t_enq - (t_zrun > 0 ? t_zrun : t_h2d)), h2d / 1e9 / std::max(t_copy - t_start, 1e-9),
-                     (unsigned long long)zjob.frames(), (unsigned long long)zjob.compressed_blocks(), (unsigned long long)zjob.sequences(), 1e3 * (t_zrun > 0 ? t_zrun - t_h2d : 0), 1e3 * (t_copy - t_enq), 1e3 * (now() - t_copy));
-    (void)all_pinned;
-    if (mode != UP_VALUES) h2d += out->nwords * 12 + nblocks * 12;
-    if (mode == UP_FULL) std::vector<DevColumn>().swap(out->h_cols);   // only a bloom-first upload needs the table again
+                     plan.arena_bytes / 1e6, h2d / 1e6, plan.layout.pieces.size(), plan.zpieces.size(), (int)!copier.staged, 1e3 * (t_desc - t_start), 1e3 * (t_alloc - t_desc), 1e3 * (t_enq - (t_zrun > 0 ? t_zrun : t_h2d)), h2d / 1e9 / std::max(t_copy - t_start, 1e-9),
+                     (unsigned long long)plan.zjob.frames(), (unsigned long long)plan.zjob.compressed_blocks(), (unsigned long long)plan.zjob.sequences(), 1e3 * (t_zrun > 0 ? t_zrun - t_h2d : 0), 1e3 * (t_copy - t_enq), 1e3 * (now() - t_copy));
+    if (headers) h2d += out->nwords * 12 + nblocks * 12;
+    if (headers && values) std::vector<DevColumn>().swap(out->h_cols);   // only a bloom-first upload needs the table again
     if (stats) stats->h2d_bytes += h2d;
 }
 
@@ -551,8 +647,18 @@ namespace {
 struct ScanRun {
     vlscan_ctx* ctx; const vlscan_program* prog; const vlscan_batch* batch;
     DevProgram P; BatchView B; std::vector<int> field_slot;   // program field -> batch field slot or -1
-    unsigned long long* stats;
+    unsigned long long* stats = nullptr;
     size_t regs_used = 0;
+    size_t slots_cursor = 0, slots_total = 0;
+
+    ScanRun(vlscan_ctx* ctx, const vlscan_program* prog, const vlscan_batch* batch) : ctx(ctx), prog(prog), batch(batch) {
+        P = const_cast<vlscan_program*>(prog)->image(ctx->device, ctx->stream);
+        B = batch->view();
+        const Program& pr = prog->p;
+        field_slot.assign(pr.fields.size(), -1);
+        for (size_t f = 0; f < pr.fields.size(); f++) for (uint32_t s = 0; s < batch->nfields; s++) if (batch->field_names[s] == pr.fields[f]) field_slot[f] = (int)s;
+        for (auto& nd : pr.nodes) slots_total += nd.prepass_count;
+    }
 
     uint64_t* new_reg() {
         if (regs_used == ctx->regs.size()) ctx->regs.emplace_back();
@@ -575,7 +681,6 @@ struct ScanRun {
                                                                              nd.kind == F_OR, reg, stats);
         launch_check(ctx);
     }
-    size_t slots_cursor = 0, slots_total = 0;
 
     void leaf(int leaf_idx, uint64_t* reg) {
         const DevLeaf& L = prog->p.leaves[leaf_idx];
@@ -727,13 +832,8 @@ static void read_stats(vlscan_ctx* ctx, vlscan_stats* st, bool check_error) {
 static void do_scan(vlscan_ctx* ctx, const vlscan_program* prog, const vlscan_batch* batch, vlscan_stats* stats) {
     VL_CUDA(cudaSetDevice(ctx->device));
     if (batch->device != ctx->device) throw BadInput("batch lives on another device than the ctx");
-    ScanRun run{ctx, prog, batch};
-    run.P = const_cast<vlscan_program*>(prog)->image(ctx->device, ctx->stream);
-    run.B = batch->view();
+    ScanRun run(ctx, prog, batch);
     const Program& pr = prog->p;
-    run.field_slot.assign(pr.fields.size(), -1);
-    for (size_t f = 0; f < pr.fields.size(); f++) for (uint32_t s = 0; s < batch->nfields; s++) if (batch->field_names[s] == pr.fields[f]) run.field_slot[f] = (int)s;
-    for (auto& nd : pr.nodes) run.slots_total += nd.prepass_count;
     uint64_t nb = std::max<uint64_t>(batch->nblocks, 1), nw = std::max<uint64_t>(batch->nwords, 1);
     ctx->action.ensure(nb); ctx->payload.ensure(nb * 8); ctx->leaf_bm.ensure(nw * 8);
     ctx->lens_blocks.ensure(nb * 4); ctx->row_blocks.ensure(nb * 4); ctx->work_count.ensure(WC_COUNT * 4);
@@ -772,13 +872,7 @@ static void do_scan(vlscan_ctx* ctx, const vlscan_program* prog, const vlscan_ba
 // batch whose values are still on the host and returns need[block * nfields + field] = 1 for every values column some filter can reach.
 static void do_probe(vlscan_ctx* ctx, const vlscan_program* prog, const vlscan_batch* batch, std::vector<uint8_t>& need) {
     VL_CUDA(cudaSetDevice(ctx->device));
-    ScanRun run{ctx, prog, batch};
-    run.P = const_cast<vlscan_program*>(prog)->image(ctx->device, ctx->stream);
-    run.B = batch->view();
-    const Program& pr = prog->p;
-    run.field_slot.assign(pr.fields.size(), -1);
-    for (size_t f = 0; f < pr.fields.size(); f++) for (uint32_t s = 0; s < batch->nfields; s++) if (batch->field_names[s] == pr.fields[f]) run.field_slot[f] = (int)s;
-    for (auto& nd : pr.nodes) run.slots_total += nd.prepass_count;
+    ScanRun run(ctx, prog, batch);
     const size_t cells = (size_t)batch->nblocks * batch->nfields;
     need.assign(cells, 0);
     if (!cells || !batch->nwords) return;
@@ -788,7 +882,7 @@ static void do_probe(vlscan_ctx* ctx, const vlscan_program* prog, const vlscan_b
     run.stats = ctx->stats.as<unsigned long long>();
     uint64_t* reg = run.new_reg();
     run.copy_reg(reg, batch->init_bitmap.as<uint64_t>());
-    run.probe_node(pr.root, reg, ctx->need.as<uint8_t>());
+    run.probe_node(prog->p.root, reg, ctx->need.as<uint8_t>());
     VL_CUDA(cudaMemcpyAsync(need.data(), ctx->need.p, cells, cudaMemcpyDeviceToHost, ctx->stream));
     VL_CUDA(cudaStreamSynchronize(ctx->stream));
 }
@@ -1062,34 +1156,28 @@ int vlscan_host_blocks_compress(const vlscan_host_blocks* in, int threads, vlsca
         std::vector<std::thread> pool; for (int t = 1; t < nt; t++) pool.emplace_back(work);
         work(); for (auto& t : pool) t.join();
         if (failed) throw BadInput(fail_msg);
-        // layout: [copied part: consts, blooms, dict tables, strided exactly like the upload arena][values blocks, back to back]
-        uint64_t cursor = 16, vbytes = 0;
-        std::vector<uint64_t> off_a(ncols, 0), off_b(ncols, 0), off_v(ncols, 0);
+        // layout: [copied part: consts, blooms, dict tables, placed as a full upload places them][values blocks, back to back]
+        ArenaLayout layout;
+        std::vector<DevColumn> at(ncols);
+        uint64_t vbytes = 0;
+        std::vector<uint64_t> off_v(ncols, 0);
         for (size_t i = 0; i < ncols; i++) {
             const vlscan_column& c = in->cols[i];
-            if (c.kind == VLSCAN_COL_CONST) { off_a[i] = arena_reserve(cursor, c.const_len); continue; }
-            off_a[i] = arena_reserve(cursor, c.bloom_len);
-            if (c.value_type == VT_DICT) off_b[i] = arena_reserve(cursor, 4 * (c.dict_len + 1) + (c.dict_len ? c.dict_offsets[c.dict_len] : 0));
-            off_v[i] = vbytes; vbytes += packed[i].size();
+            layout.put_headers(c, c.bloom_len, at[i]);
+            if (c.kind != VLSCAN_COL_CONST) { off_v[i] = vbytes; vbytes += packed[i].size(); }
         }
-        const uint64_t vbase = (cursor + kArenaPad + 63) / 64 * 64;
+        const uint64_t vbase = (layout.cursor + kArenaPad + 63) / 64 * 64;
         hb->bytes = vbase + vbytes + 64;
         VL_CUDA(cudaMallocHost(&hb->pinned, hb->bytes));
         uint8_t* base = (uint8_t*)hb->pinned;
         memset(base, 0, vbase);
+        for (const Piece& p : layout.pieces) memcpy(base + p.dst, p.src, p.len);
         hb->fields = in->fields; hb->cols = in->cols; hb->blocks = in->blocks;
         for (size_t i = 0; i < ncols; i++) {
             vlscan_column& c = hb->cols[i];
-            if (c.kind == VLSCAN_COL_CONST) { if (c.const_len) memcpy(base + off_a[i], c.const_value, c.const_len); c.const_value = base + off_a[i]; continue; }
-            if (c.bloom_len) memcpy(base + off_a[i], c.bloom, c.bloom_len);
-            c.bloom = base + off_a[i];
-            if (c.value_type == VT_DICT) {
-                uint32_t total = c.dict_len ? c.dict_offsets[c.dict_len] : 0;
-                uint8_t* m = base + off_b[i];
-                if (c.dict_len) memcpy(m, c.dict_offsets, 4 * (c.dict_len + 1)); else memset(m, 0, 4);
-                if (total) memcpy(m + 4 * (c.dict_len + 1), c.dict_blob, total);
-                c.dict_offsets = (const uint32_t*)m; c.dict_blob = m + 4 * (c.dict_len + 1);
-            }
+            if (c.kind == VLSCAN_COL_CONST) { c.const_value = base + at[i].meta_off; continue; }
+            c.bloom = base + at[i].bloom_off;
+            if (c.value_type == VT_DICT) { c.dict_offsets = (const uint32_t*)(base + at[i].meta_off); c.dict_blob = base + at[i].meta_off + 4 * (c.dict_len + 1); }
             memcpy(base + vbase + off_v[i], packed[i].data(), packed[i].size());
             c.stage = VLSCAN_STAGE_ONDISK; c.values = base + vbase + off_v[i]; c.values_len = packed[i].size();
             c.lens_items = nullptr; c.lens_items_len = 0; c.data = nullptr; c.data_len = 0;

@@ -1,5 +1,6 @@
-// Internal structures of libvlscan.so shared by vl_engine.cu (staging, scan interpreter, C ABI) and vl_gen.cu
-// (synthetic batch generator).
+// Internal structures of libvlscan.so shared by vl_engine.cu (staging, scan interpreter, C ABI), vl_gen.cu
+// (synthetic batch generator) and vl_zstd.cu.  The scan kernels (vl_kernels.cuh) are not included here: they are compiled
+// into vl_engine.cu alone.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -7,7 +8,7 @@
 #include <string>
 #include <vector>
 #include "../../include/vlscan.h"
-#include "vl_kernels.cuh"
+#include "vl_types.h"
 #include "vl_zstd.h"
 #include "vl_zstd_walk.h"   // BadInput
 #include "vl_hostpool.h"

@@ -16,6 +16,7 @@
 #include <cstring>
 #include <vector>
 #include "vl_engine.h"
+#include "vl_hd.cuh"   // fmt_u64, fmt_ipv4, ascii_tokens, xxh64
 
 using namespace vl;
 

@@ -10,28 +10,6 @@
 
 namespace vl {
 
-struct DevProgram {
-    const DevLeaf* leaves; const DevPrepass* prepass; const DevRegex* regexes;
-    const uint8_t* blob; const uint64_t* u64s; const uint32_t* u32s;
-};
-
-// stats slots (device u64 array)
-enum { ST_VALUES_BYTES = 0, ST_BLOOM_BYTES, ST_COLUMNS_READ, ST_BITMAP_BYTES, ST_ROWS_MATCHED, ST_BLOCKS_MATCHED, ST_ERROR, ST_SCAN_BYTES, ST_COUNT };
-enum { ERR_NONE = 0, ERR_LENS_MISMATCH = 1, ERR_DICT_INDEX = 2, ERR_BAD_WIDTH = 3, ERR_UNSUPPORTED_FLOAT_TOSTRING = 4, ERR_BAD_LENS_TYPE = 5, ERR_NO_TIMESTAMPS = 6, ERR_BAD_TIMESTAMPS = 7, ERR_VALUES_ABSENT = 8 };
-
-struct BatchView {
-    const uint8_t* arena;         // values payloads: lens items, data, encoded timestamps (lens_off, data_off, DevTimestamps.off)
-    const uint8_t* hdr;           // header payloads: bloom filters, const values, dict tables (bloom_off, meta_off).  The same buffer as `arena`
-                                  // unless the batch was staged bloom-first (vlscan_scan_batch): then it is the phase-1 buffer
-    const DevColumn* cols;        // [nblocks * nfields]
-    const uint32_t* blk_rows;     // [nblocks]
-    const uint64_t* blk_word_off; // [nblocks + 1]
-    const uint32_t* word_block;   // [nwords] owning block of each bitmap word
-    const DevTimestamps* ts;      // [nblocks] or NULL when the batch was staged without timestamps
-    uint32_t nblocks, nfields;
-    uint64_t nwords;
-};
-
 static __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
 #define VL_SHORT_ROW_BYTES 48u   /* average row length below which a string block is matched per row instead of row-agnostically */
 static __device__ __forceinline__ uint32_t width_of_vt(uint32_t vt) {
@@ -557,7 +535,6 @@ static __global__ void __launch_bounds__(VL_PLAN_WARPS * 32) k_plan_leaf(DevProg
 
 // ---- on-disk columns: header checks of the lens block (unmarshalUint64Items, encoding.go:246-336) once the device has regenerated it ----
 // The uint block type byte sits right in front of the lens items (lens_off - 1).  status[0] = max error code.
-struct OndiskCol { uint64_t col; uint64_t lens_total; uint64_t rows; };
 static __global__ void k_finish_ondisk_cols(const uint8_t* __restrict__ arena, DevColumn* __restrict__ cols, const OndiskCol* __restrict__ oc, uint32_t n,
                                             unsigned long long* __restrict__ status) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;

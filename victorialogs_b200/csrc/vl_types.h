@@ -1,4 +1,4 @@
-// POD layouts shared by the host program compiler (vl_program.cpp) and the CUDA engine (vl_engine.cu).
+// POD layouts shared by the host program compiler (vl_program.h), the staging code (vl_engine.h) and the CUDA kernels (vl_kernels.cuh).
 #pragma once
 #include <stdint.h>
 
@@ -114,6 +114,31 @@ struct DevPrepass {                    // one fieldTokens entry of an AND / OR n
     uint32_t tok_blob_off;
     uint32_t hashes_off, nhashes;      // u64 table
 };
+
+struct DevProgram {
+    const DevLeaf* leaves; const DevPrepass* prepass; const DevRegex* regexes;
+    const uint8_t* blob; const uint64_t* u64s; const uint32_t* u32s;
+};
+
+// stats slots (device u64 array)
+enum { ST_VALUES_BYTES = 0, ST_BLOOM_BYTES, ST_COLUMNS_READ, ST_BITMAP_BYTES, ST_ROWS_MATCHED, ST_BLOCKS_MATCHED, ST_ERROR, ST_SCAN_BYTES, ST_COUNT };
+enum { ERR_NONE = 0, ERR_LENS_MISMATCH = 1, ERR_DICT_INDEX = 2, ERR_BAD_WIDTH = 3, ERR_UNSUPPORTED_FLOAT_TOSTRING = 4, ERR_BAD_LENS_TYPE = 5, ERR_NO_TIMESTAMPS = 6, ERR_BAD_TIMESTAMPS = 7, ERR_VALUES_ABSENT = 8 };
+
+struct BatchView {
+    const uint8_t* arena;         // values payloads: lens items, data, encoded timestamps (lens_off, data_off, DevTimestamps.off)
+    const uint8_t* hdr;           // header payloads: bloom filters, const values, dict tables (bloom_off, meta_off).  The same buffer as `arena`
+                                  // unless the batch was staged bloom-first (vlscan_scan_batch): then it is the phase-1 buffer
+    const DevColumn* cols;        // [nblocks * nfields]
+    const uint32_t* blk_rows;     // [nblocks]
+    const uint64_t* blk_word_off; // [nblocks + 1]
+    const uint32_t* word_block;   // [nwords] owning block of each bitmap word
+    const DevTimestamps* ts;      // [nblocks] or NULL when the batch was staged without timestamps
+    uint32_t nblocks, nfields;
+    uint64_t nwords;
+};
+
+// An on-disk values column whose lens block the device regenerates: k_finish_ondisk_cols checks its header once it is there
+struct OndiskCol { uint64_t col; uint64_t lens_total; uint64_t rows; };
 
 enum { STR_ROW = 0, STR_SCAN = 1, STR_ALL = 2 };
 // per (block, leaf) decision of the header dispatch
